@@ -2,7 +2,7 @@
 """bench.py -- the driver's measurement contract for the ReChorus training hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c1|c2|c3|c4|c5]
-                    [--headline_only] [--no_cpu_baseline]
+                    [--headline_only] [--no_cpu_baseline] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: forward (gather + interaction), BPR loss,
 backward and the optimizer update -- the body of helpers/BaseRunner.py:193-206.  metric = training samples/s counted as
@@ -21,7 +21,11 @@ then repeats c5 alone on its GPU ("n1_same_code") so that every N>1 line carries
 Prints ONE JSON line (rank 0).  `value`: inputs already resident in HBM.  `e2e`: the same step through the public plugin
 call with the batch coming from pinned host memory every step and the loss read back every step.  `roofline`: dominant
 kernel, algorithmic bytes / CUDA-event time / measured peak.  `cpu_baseline`: the reference's own classes through its
-own BaseRunner.fit on this box's host cores (kind "reference", from baseline/_ref), else the oracle port.
+own BaseRunner.fit on this box's host cores (kind "reference", from oracle/_ref/src), else the oracle port.
+
+`--dump-outputs DIR` (c2): after the timed steps, the last timed step's results go to DIR/*.npy in float32 (see
+dump_c2_outputs).  Inputs and initial tables are seeded, so two builds run with the same arguments can be compared
+file by file.
 """
 from __future__ import annotations
 
@@ -279,6 +283,8 @@ def run_c2(args, rank, world, local_rank, sampler):
     host_ms_step = (time.time() - w0) * 1e3 / args.steps       # host time to enqueue a step (no sync inside the loop)
     dist.barrier()
     sampler.window(w0, time.time())
+    if args.dump_outputs and rank == 0:
+        dump_c2_outputs(args.dump_outputs, model, feeds[(args.warmup + args.steps - 1) % POOL], loss)
     launches = lib.b2r_launch_count() - launches0
     ms_step = dist.max_ms(t0.elapsed_time(t1)) / args.steps
     value = world * B * C / (ms_step * 1e-3)
@@ -476,6 +482,23 @@ def run_c2(args, rank, world, local_rank, sampler):
     }
 
 
+DUMP_ITEM_ROWS = 32768     # seeded sample of the last step's ~340k distinct item rows (8 MB)
+
+
+def dump_c2_outputs(dirname, model, feed, loss):
+    """What the last timed train_step returned and wrote: its loss, the user rows it updated (every distinct user of
+    the batch) and a seeded sample of the item rows it updated, in sorted id order."""
+    uu = torch.unique(feed["user_id"])
+    ii = torch.unique(feed["item_id"])
+    pick = torch.randperm(ii.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_ITEM_ROWS].sort().values
+    ii = ii[pick.to(ii.device)]
+    out = {"loss": loss.reshape(1), "user_rows": model.u_embeddings.weight.detach()[uu],
+           "item_rows": model.i_embeddings.weight.detach()[ii]}
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.float().cpu().numpy())
+
+
 def c2_self_check(model, feed, device):
     """one extra train_step verified on the device with torch formulas (fp64 gradient of the BPR objective, lazy Adam):
     a benchmark whose last step is wrong is not a benchmark"""
@@ -561,7 +584,7 @@ def run_model_steps(wname, args, rank, world, local_rank, sampler, steps_cap):
     host = make_batches(w, seed=2000 + rank, pool=4)
     feeds = [to_feed(f, device, B) for f in host]
     pinned = [to_feed(f, device, B, pin=True) for f in host]
-    steps, warmup = max(3, min(args.steps, steps_cap)), max(3, min(args.warmup, 5))
+    steps, warmup = min(args.steps, steps_cap), max(3, min(args.warmup, 5))
 
     def step(k):
         f = feeds[k % len(feeds)]
@@ -712,7 +735,7 @@ def run_c5(args, rank, world, local_rank, sampler, steps_cap, group=None, solo=F
             for _ in range(4)]
     pool = [(u.to(device), i.to(device)) for u, i in host]
     pinned = [(u.pin_memory(), i.pin_memory()) for u, i in host]
-    steps, warmup = max(3, min(args.steps, steps_cap)), max(3, min(args.warmup, 5))
+    steps, warmup = min(args.steps, steps_cap), max(3, min(args.warmup, 5))
     launches0 = lib.b2r_launch_count()
     ms, loss, win = timed_loop(dist, lambda k: m.train_step(*pool[k % 4]), steps, warmup)
     launches = lib.b2r_launch_count() - launches0
@@ -835,7 +858,11 @@ def main():
     ap.add_argument("--workload", type=str, default="", choices=[""] + sorted(WORKLOADS))
     ap.add_argument("--no_cpu_baseline", action="store_true", help="skip the CPU legs (dev runs)")
     ap.add_argument("--headline_only", action="store_true", help="N=1: only the headline workload, no per-config block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="c2: write the last timed step's loss and updated table rows to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -844,6 +871,8 @@ def main():
     explicit = bool(args.workload)
     if not args.workload:
         args.workload = "c2" if max(world, args.gpus) == 1 else "c5"
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs covers the c2 workload of --impl ours")
 
     if args.impl == "reference":
         out = run_reference_arm(args, rank)

@@ -1,6 +1,6 @@
 """Run the reference's UNCHANGED ``src/main.py`` with the kernel-backed model classes substituted.
 
-    python -m rechorus_b200.overlay --ref /root/reference/src --model_name BPRMF --emb_size 64 --lr 1e-3 \
+    python -m rechorus_b200.overlay --ref <ReChorus>/src --model_name BPRMF --emb_size 64 --lr 1e-3 \
         --l2 1e-6 --dataset Grocery_and_Gourmet_Food --path /tmp/data/ [--table_mode fused]
 
 What it does (SURVEY.md section 8b1): puts the reference ``src/`` on ``sys.path``, restores the NumPy aliases the
@@ -10,8 +10,8 @@ reference's Dataset, reader, runner, argument plumbing and checkpoint code are t
 ``models.general.BPRMF.BPRMF`` etc. with them, and ``runpy``s ``main.py``.  With ``--fused_step 1`` or
 ``--device_metrics 1`` on the command line it also registers ``helpers.B200Runner`` (a subclass of the reference's own
 BaseRunner) through the same by-name discovery.  Needs a CUDA device for the first forward call; there is no CPU
-fallback.  ``--ref`` defaults to /root/reference/src, or to the copy tools/install_reference.py ships in
-baseline/_ref/src (the GPU box has no /root/reference).
+fallback.  ``--ref`` (a ReChorus ``src/`` directory) defaults to the ``RECHORUS_SRC`` environment variable, else to the
+unmodified copy build() places in oracle/_ref/src.
 """
 from __future__ import annotations
 
@@ -19,9 +19,8 @@ import os
 import runpy
 import sys
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_SHIPPED = os.path.join(os.path.dirname(_HERE), "baseline", "_ref", "src")      # tools/install_reference.py
-DEFAULT_REF = "/root/reference/src" if os.path.isdir("/root/reference/src") else _SHIPPED
+DEFAULT_REF = os.environ.get("RECHORUS_SRC") or os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
+                                                           "oracle", "_ref", "src")
 
 
 def _make_runner_module(ref_runner_cls):
@@ -185,6 +184,8 @@ def main(argv=None):
         i = argv.index("--ref")
         ref = argv[i + 1]
         del argv[i:i + 2]
+    if not os.path.isfile(os.path.join(ref, "main.py")):
+        sys.exit("rechorus_b200.overlay: no ReChorus main.py under %r (pass --ref <ReChorus>/src or set RECHORUS_SRC)" % ref)
     # the runner seams only matter when one of their flags is on the command line; otherwise the reference's own
     # BaseRunner class is the one main.py instantiates
     want_runner = any(a in ("--fused_step", "--device_metrics") or a.startswith(("--fused_step=", "--device_metrics="))

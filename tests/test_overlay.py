@@ -1,5 +1,5 @@
-"""CPU, build container only: the overlay drives the reference's unchanged main.py up to the first forward,
-where the kernel-backed class refuses to run without CUDA (no CPU fallback)."""
+"""CPU, where build() placed the unmodified reference in oracle/_ref (rechorus_b200.overlay.DEFAULT_REF): the overlay
+drives the reference's unchanged main.py up to the first forward, where the kernel-backed class refuses to run without CUDA (no CPU fallback)."""
 import os
 import subprocess
 import sys
@@ -8,10 +8,12 @@ import numpy as np
 import pandas as pd
 import pytest
 
-REF = "/root/reference/src"
+from rechorus_b200.overlay import DEFAULT_REF as REF
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "main.py")),
+                                reason="no ReChorus sources: build() found no checkout to place in oracle/_ref")
 
 
 def _tiny_dataset(root):
@@ -33,7 +35,7 @@ def test_reference_main_runs_our_class_and_refuses_cpu(tmp_path, model):
     path = _tiny_dataset(str(tmp_path))
     src = tmp_path / "src"          # main.py writes ../log and ../model relative to the cwd
     src.mkdir()
-    cmd = [sys.executable, "-m", "rechorus_b200.overlay", "--model_name", model, "--dataset", "tiny", "--path", path,
+    cmd = [sys.executable, "-m", "rechorus_b200.overlay", "--ref", REF, "--model_name", model, "--dataset", "tiny", "--path", path,
            "--gpu", "", "--num_workers", "0", "--epoch", "1", "--emb_size", "64", "--history_max", "5"]
     env = dict(os.environ, PYTHONPATH=ROOT)
     res = subprocess.run(cmd, cwd=str(src), env=env, capture_output=True, text=True, timeout=300)

@@ -1,8 +1,8 @@
 """CPU reference legs of bench.py: the reference's OWN classes driven by its OWN ``BaseRunner.fit`` on a bounded synthetic
 corpus (kind "reference"), or -- where the unmodified reference is not on the box -- the oracle port (kind "port").
 
-The reference tree is looked up at /root/reference/src (build container) or baseline/_ref/src (the copy
-tools/install_reference.py ships to the GPU box).  Nothing of rechorus_b200 is imported here: this is the arm the product
+The reference tree is the ``src/`` directory the RECHORUS_SRC environment variable names, else the unmodified copy
+build() places in oracle/_ref/src.  Nothing of rechorus_b200 is imported here: this is the arm the product
 is compared against.  ``oracle/`` is touched only by the "port" fallback (bench.py's cpu_baseline contract)."""
 from __future__ import annotations
 
@@ -19,10 +19,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def reference_src():
-    for p in ("/root/reference/src", os.path.join(ROOT, "baseline", "_ref", "src")):
-        if os.path.isfile(os.path.join(p, "main.py")):
-            return p
-    return None
+    p = os.environ.get("RECHORUS_SRC") or os.path.join(ROOT, "oracle", "_ref", "src")
+    return p if os.path.isfile(os.path.join(p, "main.py")) else None
 
 
 def use_all_host_threads() -> int:

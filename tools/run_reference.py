@@ -1,5 +1,6 @@
 #!/usr/bin/env python
-"""Run the UNMODIFIED reference main.py (baseline/_ref/src or /root/reference/src) on today's NumPy.
+"""Run the UNMODIFIED reference main.py (``--ref``, the RECHORUS_SRC environment variable, else the copy build() places
+in oracle/_ref/src) on today's NumPy.
 
     python tools/run_reference.py [--ref DIR] <main.py arguments>
 
@@ -17,7 +18,7 @@ HERE = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 def main():
     argv = sys.argv[1:]
-    ref = "/root/reference/src" if os.path.isdir("/root/reference/src") else os.path.join(HERE, "baseline", "_ref", "src")
+    ref = os.environ.get("RECHORUS_SRC") or os.path.join(HERE, "oracle", "_ref", "src")
     if "--ref" in argv:
         i = argv.index("--ref")
         ref = argv[i + 1]
